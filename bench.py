@@ -63,6 +63,8 @@ SUB_WORKLOADS = ["cfg2-random", "cfg-self", "cfg3", "cfg4", "cfg5"]
 # decisions of the queue's head the CPU reference is run on (parity + cpu_baseline), sized for a few seconds each
 CPU_SAMPLE = {"cfg1": 1000, "cfg2-mod": 100_000, "cfg2-random": 100_000, "cfg-self": 100_000, "cfg3": 100_000,
               "cfg4": 100_000, "cfg5": 50_000}
+# --dump-outputs: grants per array at most; a longer queue is sampled at fixed, seeded positions (7 float64 arrays, ~30 MB)
+DUMP_CAP = 1 << 19
 
 
 def build_workload(name: str, rank: int = 0):
@@ -261,7 +263,9 @@ def grants_equal(a: np.ndarray, b: np.ndarray) -> bool:
 # one workload on the GPU
 # ---------------------------------------------------------------------------------------------
 
-def measure_workload(name: str, dev_index: int, steps: int, warmup: int, solver: int, with_cpu: bool, flush, sampler=None):
+def measure_workload(name: str, dev_index: int, steps: int, warmup: int, solver: int, with_cpu: bool, flush, sampler=None,
+                     keep_last: bool = False):
+    """keep_last: extra["last_grants"] = the grants of the last timed step's e2e call and staged solve."""
     import torch
 
     w = build_workload(name)
@@ -323,6 +327,7 @@ def measure_workload(name: str, dev_index: int, steps: int, warmup: int, solver:
     dev_ms, e2e_ms, e2e24_ms, launches, n_solves = [], [], [], 0, 0
     granted = h2d = d2h = h2d24 = d2h24 = solver_used = offered = 0
     prev_ids = None
+    last_grants = {}
     t_wall0 = time.perf_counter()
     for it in range(warmup + steps):
         now = 2.0 + it
@@ -343,6 +348,8 @@ def measure_workload(name: str, dev_index: int, steps: int, warmup: int, solver:
         st = d.last_solve_stats()
         if use_packed:
             g = unpack_grants(g[0], g[1])  # (untimed: the caller's id arithmetic, done here for the FreeTask below)
+        if keep_last and it == warmup + steps - 1:
+            last_grants["e2e"] = g.copy()
         ok = g["status"] == STATUS_GRANTED
         prev_ids = g["task_id"][ok].copy()
         granted = int(ok.sum())
@@ -380,6 +387,8 @@ def measure_workload(name: str, dev_index: int, steps: int, warmup: int, solver:
         g, _ = one_pass(src if stages is not None else reqs, now, "staged")
         t1 = time.perf_counter()
         st = d.last_solve_stats()
+        if keep_last and it == warmup + steps - 1:
+            last_grants["staged"] = g.copy()
         ok = g["status"] == STATUS_GRANTED
         prev_ids = g["task_id"][ok].copy()
         assert int(ok.sum()) == granted
@@ -416,8 +425,22 @@ def measure_workload(name: str, dev_index: int, steps: int, warmup: int, solver:
                                "h2d_bytes_per_step": int(h2d24), "d2h_bytes_per_step": int(d2h24),
                                "call": "yd_wait_for_starting_new_tasks (24-byte requests, 16-byte grants)"}
     extra = {"e2e_ms": e2e_ms, "dev_ms": dev_ms, "launches": launches, "n_solves": n_solves, "wall": wall,
-             "S": S_count, "n": n, "w": w}
+             "S": S_count, "n": n, "w": w, "last_grants": last_grants}
     return rec, extra
+
+
+def dump_outputs(directory: str, last_grants: dict) -> None:
+    """<call>_<field>.npy (float64) for each call's grants; sample_index.npy holds the positions kept when a queue
+    is longer than DUMP_CAP."""
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    for call, g in last_grants.items():
+        idx = np.arange(len(g))
+        if len(g) > DUMP_CAP:
+            idx = np.sort(np.random.default_rng(0).choice(len(g), DUMP_CAP, replace=False))
+            np.save(out / "sample_index.npy", idx.astype(np.float64))
+        for field in ("status", "servant_index", "task_id"):
+            np.save(out / f"{call}_{field}.npy", g[field][idx].astype(np.float64))
 
 
 def latency_sweep(dev_index: int, sizes=(1, 32, 1024), reps=200):
@@ -502,7 +525,10 @@ def run_ours(args):
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)  # > 126 MB L2
     sampler = ClockSampler(local)
-    rec, ex = measure_workload(args.workload, local, args.steps, args.warmup, args.solver, not args.no_cpu_baseline, flush, sampler)
+    rec, ex = measure_workload(args.workload, local, args.steps, args.warmup, args.solver, not args.no_cpu_baseline, flush, sampler,
+                               keep_last=args.dump_outputs is not None)
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, ex["last_grants"])
     sampler.stop_flag.set()
     sampler.join(timeout=2)
     if rec["parity_in_run"] is False:
@@ -597,9 +623,12 @@ def main():
     ap.add_argument("--solver", type=int, default=0, help="0 auto, 1 row-scan, 2 slot-stream")
     ap.add_argument("--sub", default="all", help="sub-records beside the headline: all | none | comma-separated workloads")
     ap.add_argument("--sub-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's grants of the headline workload to DIR/*.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
+    if args.dump_outputs is not None and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs covers the single-GPU CUDA run only")
     if args.impl == "reference":
         run_reference(args)
     else:

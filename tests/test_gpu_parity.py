@@ -8,7 +8,6 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from conftest import REF_LIB
 from golden_cases import ALL_CASES
 from yadcc_b200 import streams as S
 from yadcc_b200 import STATUS_GRANTED
@@ -42,7 +41,7 @@ def _parity(make_dispatcher, name_or_builder, kinds=("port",), solver=0):
 @pytest.mark.parametrize("solver", [0, 1, 2], ids=SOLVERS.get)
 @pytest.mark.parametrize("seed", range(150))
 def test_fuzz_cuda_equals_oracle(make_dispatcher, seed, solver):
-    kinds = ("port", "ref") if REF_LIB.exists() and seed % 3 == 0 else ("port",)
+    kinds = ("port", "ref") if seed % 3 == 0 else ("port",)
     _parity(make_dispatcher, lambda d: S.fuzz_stream(d, seed, n_servants=8 + seed % 30, wide=(seed % 5 == 0)), kinds,
             solver)
 
@@ -172,7 +171,7 @@ def test_fuzz_one_daemon_per_machine(make_dispatcher, seed, merge_self):
     """Every servant on its own IP and many requestors that are servants: the merge solver's own-servant
     rule, passed-over (pending) requests and -- capacity is tiny here -- the last-resort hand-back to the
     sequential solver all get exercised; every third seed also against the reference itself."""
-    kinds = ("port", "ref") if REF_LIB.exists() and seed % 3 == 0 else ("port",)
+    kinds = ("port", "ref") if seed % 3 == 0 else ("port",)
     traces = {}
     for kind in ("cuda",) + kinds:
         d = make_dispatcher(kind, merge_self=merge_self) if kind == "cuda" else make_dispatcher(kind)
@@ -268,7 +267,7 @@ def test_dump_internals_on_cuda(make_dispatcher, seed):
     """DumpInternals (task_dispatcher.cc:538-614): per-servant rows and summary of the CUDA backend against the
     reference's own function after the same stream."""
     dumps = []
-    for kind in ("cuda", "ref" if REF_LIB.exists() else "port"):
+    for kind in ("cuda", "ref"):
         d = make_dispatcher(kind)
         S.Replayer(d).run(S.fuzz_stream(d, seed, n_servants=12 + seed))
         dumps.append(d.dump_internals())
@@ -481,9 +480,8 @@ def test_rpc_expansion_cuda_equals_oracle(make_dispatcher, seed):
     scheduler_service_impl.cc:209-271) on the CUDA backend against the oracle."""
     from rpc_cases import run_rpc_stream
 
-    ref = "ref" if REF_LIB.exists() else "port"
     a = run_rpc_stream(make_dispatcher("cuda"), seed)
-    b = run_rpc_stream(make_dispatcher(ref), seed)
+    b = run_rpc_stream(make_dispatcher("ref"), seed)
     for x, y in zip(a, b):
         assert x.shape == y.shape and (x == y).all()
 
@@ -540,9 +538,8 @@ def test_bloom_prefilter_cuda_equals_oracle(make_dispatcher, seed):
     all key lengths, tiny geometries, imported filters."""
     from bloom_cases import run_bloom_suite
 
-    ref = "ref" if REF_LIB.exists() else "port"
     a = run_bloom_suite(make_dispatcher("cuda"), seed)
-    b = run_bloom_suite(make_dispatcher(ref), seed)
+    b = run_bloom_suite(make_dispatcher("ref"), seed)
     assert len(a) == len(b)
     for k, (x, y) in enumerate(zip(a, b)):
         assert x.shape == y.shape and (x == y).all(), k

@@ -21,8 +21,9 @@ def _same(a, b):
 
 
 @pytest.mark.parametrize("case", CASES, ids=lambda c: c.__name__)
-def test_service_case(make_dispatcher, case):
+def test_service_case(make_dispatcher, reference, case):
     a = case(make_dispatcher("ref"))
+    reference.observe(a)
     b = case(make_dispatcher("port"))
     assert _same(a, b)
 

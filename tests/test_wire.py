@@ -8,8 +8,9 @@ pytest.importorskip("google.protobuf")
 from wire_cases import run_wire_scenario
 
 
-def test_wire_scenario_port_equals_reference(make_dispatcher):
+def test_wire_scenario_port_equals_reference(make_dispatcher, reference):
     a = run_wire_scenario(make_dispatcher, "ref")
+    reference.observe(a)
     b = run_wire_scenario(make_dispatcher, "port")
     assert a == b
 
@@ -80,7 +81,7 @@ def test_wire_parser_survives_mutated_frames(make_dispatcher):
     assert min(verdicts.values()) > 100  # all three outcomes really occurred
 
 
-def test_wire_request_counts_are_not_trusted(make_dispatcher):
+def test_wire_request_counts_are_not_trusted(make_dispatcher, reference):
     """immediate_reqs / prefetch_reqs are uint32s off the wire.  A caller with a BAD token and
     immediate_reqs = 0xFFFFFFFF gets ACCESS_DENIED (scheduler_service_impl.cc:216-219) before
     anything is sized for it; a caller with a good token gets exactly what the reference's loop
@@ -116,4 +117,5 @@ def test_wire_request_counts_are_not_trusted(make_dispatcher):
         out = svc.handle_frames(frames, now=1.5)
         assert [o[2] for o in out] == [1003, 1001]  # the pool is full now: NO_QUOTA for the good caller
         svc.close()
+    reference.observe(results[1])
     assert results[0] == results[1]
