@@ -1176,6 +1176,16 @@ uint64_t NextPow2(uint64_t v, uint64_t lo) {
   return r;
 }
 
+// Largest grid (1024-request blocks) whose slot-stream final is the one-launch k_final_fused: beyond ~2 M requests the
+// look-back chain of 1024-thread blocks is slower than three plain passes (count, scan, write).
+constexpr uint32_t kFinalFusedMaxBlocks = 2048;
+
+// Kernels that write the grants after the solver: 0 (the solo fused kernel wrote them), 1 (k_final_fused) or 3.
+uint32_t FinalPasses(bool solo, uint32_t solver, bool have_work, uint32_t nb) {
+  if (solo) return 0;
+  return solver == 2 && have_work && nb <= kFinalFusedMaxBlocks ? 1 : 3;
+}
+
 // Everything between the request upload and the grant download, for size class
 // (Nb, slot_b): the sequence that is captured into a CUDA graph.
 // variant: 0 = the kernel-by-kernel pipeline, 1 = fused front + coupled solvers + final, 2 = fused front alone (solo).
@@ -1226,11 +1236,11 @@ uint32_t EnqueueSolve(yd_sched* s, uint32_t Nb, size_t slot_b, uint32_t solver, 
     if (have_work) launches += LaunchRowscan(s);
   }
   if (record_events) YD_CUDA_CHECK(cudaEventRecord(s->ev[3], st));
-  if (solo) {
+  const uint32_t final_passes = FinalPasses(solo, solver, have_work, nb);
+  if (final_passes == 0) {
     // grants, ids and leases were written by the fused kernel
-  } else if (solver == 2 && have_work && nb <= 2048) {
-    // grants, task ids (single-pass scan with look-back), leases, ++running_tasks: one launch (beyond ~2 M requests the
-    // look-back chain of 1024-thread blocks is slower than three plain passes)
+  } else if (final_passes == 1) {
+    // grants, task ids (single-pass scan with look-back), leases, ++running_tasks: one launch
     unsigned long long* look = reinterpret_cast<unsigned long long*>(static_cast<char*>(s->d_zero.p) + s->z_final_off);
     yd::k_final_fused<<<nb, 1024, 0, st>>>(s->d_res.as<uint32_t>(), s->d_reqs.as<yd_task_req>(), dp, look, nb,
                                            s->d_comp_sv.as<uint32_t>(), s->ring(), s->d_out.as<yd_grant>(),
@@ -1485,6 +1495,8 @@ void WaitImpl(yd_sched* s, int64_t now_ns, const yd_task_req* reqs, const yd_tas
   void* const out_dev = mapped_address(out ? static_cast<void*>(out) : static_cast<void*>(out8));
   if (in_host) s->staged_n = 0;  // the staging area now holds this batch
   bool graphed = false;
+  size_t fused_dyn = 0;  // dynamic shared memory of the solo fused kernel (0: its list offsets are read from HBM)
+  uint32_t variant_ran = 0;  // the fused variant of the pass that decided the batch
   const uint32_t merge_rounds_cfg = s->merge_rounds, force_stream_cfg = s->force_stream;
   int merge_retry = 0, grow_attempts = 0;
   for (;;) {
@@ -1581,6 +1593,7 @@ void WaitImpl(yd_sched* s, int64_t now_ns, const yd_task_req* reqs, const yd_tas
         np.extra = nullptr;
         YD_CUDA_CHECK(cudaGraphExecKernelNodeSetParams(hit->exec, hit->knode, &np));
       }
+      fused_dyn = variant >= 2 ? hit->fdyn : 0;
       hp[3] = hp_now();
       YD_CUDA_CHECK(cudaEventRecord(s->ev[1], st));
       YD_CUDA_CHECK(cudaGraphLaunch(hit->exec, st));
@@ -1594,6 +1607,7 @@ void WaitImpl(yd_sched* s, int64_t now_ns, const yd_task_req* reqs, const yd_tas
         launches += RebuildSlotOrder(s, slot_b);
       }
       launches += EnqueueSolve(s, Nb, slot_b, solver, true, false, variant, packed);
+      fused_dyn = variant >= 2 ? s->last_fused_dyn : 0;
     }
     if (solver == 1) { s->order_dirty = true; s->order_static = false; }  // the row-scan solver's table overwrote the kept one
     if (zc_out) {}  // the kernel wrote the grants into the caller's page-locked array
@@ -1662,6 +1676,7 @@ void WaitImpl(yd_sched* s, int64_t now_ns, const yd_task_req* reqs, const yd_tas
       s->clean_sig = sig_now;
       s->clean_valid = true;
     }
+    variant_ran = variant;
     break;
   }
   const Counters* c = s->h_counters.as<Counters>();
@@ -1686,8 +1701,12 @@ void WaitImpl(yd_sched* s, int64_t now_ns, const yd_task_req* reqs, const yd_tas
             hp[1] - hp[0], hp[2] - hp[1], hp[3] - hp[2], hp[4] - hp[3], hp[5] - hp[4], hp[6] - hp[5], hp[7] - hp[6], hp[7] - hp[0]);
   }
   if (s->debug_env) {
-    fprintf(stderr, "ydsched: solver %u graph %d merge_rounds %llu merge_chunks %llu walks %llu windows %llu solve_ms %.3f\n",
-            solver, (int)graphed, c->pad[0], c->pad[1], c->pad[2], c->pad[3], stt.solve_ms);
+    // (which path decided the batch: fused variant (0 = pipeline, 1 = front + coupled solvers, 2/3 = solo), the solo
+    // kernel's shared-memory offset table, the final's launches, 64-bit slot keys, the kept slot table)
+    fprintf(stderr, "ydsched: solver %u graph %d merge_rounds %llu merge_chunks %llu walks %llu windows %llu solve_ms %.3f"
+            " variant %u fused_dyn %zu lite %d final_passes %u wide %d static %d\n",
+            solver, (int)graphed, c->pad[0], c->pad[1], c->pad[2], c->pad[3], stt.solve_ms, variant_ran, fused_dyn,
+            (int)s->fused_lite, FinalPasses(variant_ran >= 2, solver, S && s->n_comps, nb), (int)s->wide, (int)want_static);
   }
 }
 }  // namespace
